@@ -2,7 +2,7 @@
 """bench.py -- SpMM aggregated-edges/s and HBM GB/s (hidden=128) on synthetic power-law CSR graphs.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--no-extras]
-                  [--beta B] [--scaling weak|strong]
+                  [--beta B] [--scaling weak|strong] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one pass of the hot path over one synthetic graph:
@@ -55,6 +55,7 @@ FLUSH_BYTES = 512 << 20
 METRIC = "spmm_aggregated_edges_per_sec"
 CPU_SLICE_EDGES = 12_000_000      # reference arm at N > 1: leading row slice of rank 0's shard
 PARITY_ROWS = 4096
+DUMP_ROWS = 1 << 16               # --dump-outputs: at most 32 MiB of sampled output rows (hidden=128, fp32)
 
 
 def load_synth():
@@ -294,8 +295,9 @@ def cpu_baseline_leg(rp, col, w, x, nnz):
 
 
 # --------------------------------------------------------------------------------------------- our arm
-def time_steps(fn, steps, warmup, flush, torch, dist_on):
-    """Per-step CUDA-event intervals (ms), L2 flushed between steps; max over ranks per step."""
+def time_steps(fn, steps, warmup, flush, torch, dist_on, keep_last=False):
+    """Per-step CUDA-event intervals (ms), L2 flushed between steps; max over ranks per step.
+    keep_last: also return what the last timed step computed, as (ms, output)."""
     for _ in range(warmup):
         fn()
     torch.cuda.synchronize()
@@ -303,12 +305,16 @@ def time_steps(fn, steps, warmup, flush, torch, dist_on):
         import torch.distributed as dist
         dist.barrier()
     evs = []
-    for _ in range(steps):
+    last = None
+    for i in range(steps):
         if flush is not None:
             flush.zero_()       # evicts X / Y from the 126 MB L2; outside the timed interval
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
-        fn()
+        if keep_last and i == steps - 1:
+            last = fn()
+        else:
+            fn()
         b.record()
         evs.append((a, b))
     torch.cuda.synchronize()
@@ -319,7 +325,7 @@ def time_steps(fn, steps, warmup, flush, torch, dist_on):
     if dist_on:
         import torch.distributed as dist
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-    return ms.cpu().tolist()
+    return (ms.cpu().tolist(), last) if keep_last else ms.cpu().tolist()
 
 
 def time_e2e(torch, dev, x_pin, x_in, run, n_rows, steps, warmup, dist_on, before_h2d=None):
@@ -388,6 +394,20 @@ def bind_to_gpu_numa(torch, local):
         return {"numa_node": node, "cpus": len(cpus), "pci": bdf}
     except Exception as ex:  # noqa: BLE001
         return {"numa_node": None, "note": f"{type(ex).__name__}: {ex}"}
+
+
+def dump_output(out_dir, name, y, max_rows):
+    """--dump-outputs: `y` (rows x F) as out_dir/<name>.npy in float32.  Above `max_rows` rows, a fixed seeded
+    sample of rows in ascending order, with their indices as out_dir/<name>_rows.npy (float64)."""
+    import numpy as np
+    import torch
+
+    os.makedirs(out_dir, exist_ok=True)
+    if y.shape[0] > max_rows:
+        rows = torch.randperm(y.shape[0], generator=torch.Generator().manual_seed(0))[:max_rows].sort().values
+        np.save(os.path.join(out_dir, name + "_rows.npy"), rows.double().numpy())
+        y = y[rows.to(y.device)]
+    np.save(os.path.join(out_dir, name + ".npy"), y.float().cpu().numpy())
 
 
 def elementwise_err(got, ref):
@@ -738,9 +758,12 @@ def run_ours(args):
         # ---- device-resident
         l0 = _cabi.launch_count()
         sampler.start()
-        ms = time_steps(step, args.steps, args.warmup, flush, torch, False)
+        ms, y_last = time_steps(step, args.steps, args.warmup, flush, torch, False, keep_last=True)
         launches_dev = _cabi.launch_count() - l0
         kernel_name = _cabi.last_kernel()
+        if args.dump_outputs:
+            dump_output(args.dump_outputs, "spmm_out", y_last, DUMP_ROWS)
+        del y_last
         # ---- parity of what was just timed, against the oracle (outside the timed regions)
         parity = parity_single(torch, rp, col, w, x_host, step(), st.chunk_edges)
         # ---- end to end: pinned host X -> device, spmm through the public API, Y -> pinned host
@@ -768,10 +791,13 @@ def run_ours(args):
         phases["setup_s"] = time.perf_counter() - t_begin
         l0 = _cabi.launch_count()
         sampler.start()
-        ms = time_steps(step, args.steps, args.warmup, flush, torch, True)
+        ms, y_last = time_steps(step, args.steps, args.warmup, flush, torch, True, keep_last=True)
         clocks = sampler.stop()
         launches_dev = _cabi.launch_count() - l0
         kernel_name = _cabi.last_kernel()
+        if args.dump_outputs:     # this rank's rows of the output
+            dump_output(args.dump_outputs, f"spmm_out_rank{rank}", y_last, DUMP_ROWS // world)
+        del y_last
         t0 = time.perf_counter()
         parity = parity_dist(torch, part, step(), dev)
         phases["parity_s"] = time.perf_counter() - t0
@@ -858,7 +884,7 @@ def run_ours(args):
         if not args.no_extras:
             del g, st, x_dev, x_in
             torch.cuda.empty_cache()
-            line["others"] = extras(torch, flush, synth)
+            line["others"] = extras(torch, flush, synth, args.steps)
     phases["total_s"] = time.perf_counter() - t_begin
     line["phases"] = phases
     if rank == 0:
@@ -883,6 +909,9 @@ def main():
                     help="N > 1: probability that a column is drawn over the whole graph instead of the own node range")
     ap.add_argument("--scaling", default=os.environ.get("COGDL_B200_DIST_SCALING", "weak"), choices=["weak", "strong"],
                     help="N > 1: weak = 1/8 of papers100M per GPU; strong = papers100M split N ways")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output of the last one to DIR/*.npy (a fixed seeded row "
+                         "sample when larger than %d rows) so that two builds can be compared" % DUMP_ROWS)
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
     if args.impl == "reference":

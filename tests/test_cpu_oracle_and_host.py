@@ -11,6 +11,7 @@ import pytest
 import torch
 
 import oracle
+from tests import refgold
 from tests.graphs import CASES, case
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -67,18 +68,13 @@ def test_oracle_gat_forward_vs_reference_gat_layer():
 
 
 # ------------------------------------------------------------------ oracle vs the reference's own compiled C++
+# (its outputs stored as digests in tests/golden/ops_digests.json by tests/golden/make_golden_ops.py)
 @pytest.mark.parametrize("variant", ["asis", "o3"])
 @pytest.mark.parametrize("name", [k for k in CASES if k != "rect"])
 def test_oracle_spmm_bit_exact_vs_compiled_reference(variant, name):
-    if not oracle.ref_available("spmm_cpu", variant):
-        pytest.skip("oracle/_ref not built (needs /root/reference)")
-    fn = oracle.ref_module("spmm_cpu", variant).csr_spmm_cpu
-    rp, ci, n_cols = case(name)
-    rng = np.random.default_rng(0)
-    X = rng.standard_normal((n_cols, 48)).astype(np.float32)
-    val = rng.random(ci.shape[0]).astype(np.float32)
-    ref = fn(torch.from_numpy(rp), torch.from_numpy(ci), torch.from_numpy(val), torch.from_numpy(X)).numpy()
-    assert np.array_equal(oracle.spmm_csr(rp, ci, val, X), ref)
+    rp, ci, val, X = refgold.spmm_cpu_inputs(name)
+    got = refgold.digest(oracle.spmm_csr(rp, ci, val, X), np.float32)
+    assert got == refgold.expected_digest(f"spmm_cpu/{variant}/{name}")
 
 
 def test_oracle_csr2csc_is_stable_transpose():
@@ -265,25 +261,18 @@ def test_install_registers_backend_in_reference_package():
 
 def test_oracle_sampler_is_pinned_to_the_reference_sample_cpp():
     """No-randomness paths of sample.cpp (sample_adj with num_neighbors = -1, subgraph) compiled from the
-    reference's own source (oracle/_ref) vs the oracle restatement: every output array identical."""
-    if not oracle.ref_available("sampler", "asis"):
-        pytest.skip("oracle/_ref not built")
-    smp = oracle.ref_module("sampler", "asis")
+    reference's own source vs the oracle restatement: every output array identical (the reference's outputs
+    stored as digests in tests/golden/ops_digests.json)."""
     rng = np.random.default_rng(0)
-    for n, hi in ((500, 12), (3000, 40), (40, 3)):
-        deg = rng.integers(0, hi, n)
-        indptr = np.zeros(n + 1, np.int64)
-        indptr[1:] = np.cumsum(deg)
-        indices = rng.integers(0, n, int(indptr[-1])).astype(np.int64)
-        batch = rng.permutation(n)[: max(1, n // 6)].astype(np.int64)
-        t = [torch.from_numpy(a) for a in (indptr, indices, batch)]
-        ref = smp.sample_adj(t[0], t[1], t[2], -1, False)
+    for n, hi in refgold.SAMPLER_SHAPES:
+        indptr, indices, batch = refgold.sampler_inputs(rng, n, hi)
         got = oracle.sample_adj(indptr, indices, batch, -1, False)
-        assert all(np.array_equal(a.numpy(), b) for a, b in zip(ref, got))
-        ref = smp.subgraph(t[0], t[1], t[2])
+        assert len(got) == 4
+        for k, a in enumerate(got):
+            assert refgold.digest(a, np.int64) == refgold.expected_digest(f"sample_adj/{n}/{k}"), (n, k)
         got = oracle.subgraph(indptr, indices, batch)
-        assert np.array_equal(ref[0].numpy(), got[0]) and np.array_equal(ref[1].numpy(), got[1])
-        assert np.array_equal(ref[3].numpy(), got[2]) and np.array_equal(ref[2].numpy(), np.arange(batch.shape[0]))
+        for k, a in ((0, got[0]), (1, got[1]), (2, np.arange(batch.shape[0])), (3, got[2])):
+            assert refgold.digest(a, np.int64) == refgold.expected_digest(f"subgraph/{n}/{k}"), (n, k)
         # random paths: the row sizes and the first-appearance numbering obey the reference's rules
         for size, replace in ((4, True), (4, False)):
             oi, oc, on, oe = oracle.sample_adj(indptr, indices, batch, size, replace, seed=7)
